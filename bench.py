@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — mel-frames/sec of the E2-TTS flow-matching hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--dropout P]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--dropout P] [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`):
   2 (default, the metric's config)  E2TTS(dim 512, depth 8, heads 8, 100 mels) forward + loss.backward(), per-GPU batch 16 x 1024 frames
@@ -20,10 +20,18 @@ One JSON line is printed by rank 0 (contract: see DESIGN.md §measurement):
                 BASELINE cfg1 exactly (B = 2 x 1024 frames, same d512 / depth-8 model): 2 warm-up + 5 timed steps, median
 `--impl reference` times that CPU path alone (the reference itself is pure Python + unvendored deps and cannot travel
 to the GPU box; see DESIGN.md).
+`--dump-outputs DIR` writes, after the timed steps, what the last step of the timed path (the one `value` reports) returned to its
+caller, as float32 .npy files: for training steps `loss`, `grad_norms` (the norm of every parameter's gradient, in
+model.parameters() order) and `grads_sample` (a fixed seeded sample of 2^23 entries of all gradients concatenated in that order),
+for cfg5 the generated mel frames `mel`. Weights (torch and Python's random module), inputs and random draws are seeded, so the files
+of two builds compare entry for entry. Two runs of one build agree to the last bits only: some kernels (loss sums, bias and gain
+gradients, hyper-connection backward) accumulate with float atomics, whose order varies from run to run; on a B200 (1000 W) two cfg2
+runs gave the same loss and gradients within 2e-7 of each other (largest entry 0.024).
 """
 import argparse
 import json
 import os
+import random
 import subprocess
 import sys
 import threading
@@ -31,6 +39,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the tree as it found it (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -126,9 +135,11 @@ def run_cpu(steps, warmup, budget_s=150.0, threads=None):
 
 
 def run_cpu_bounded(steps, warmup, timeout_s):
-    """Run the CPU leg in a child process with a hard wall-clock bound, so that a slow host can never cost the GPU line."""
+    """Run the CPU leg in a child process with a hard wall-clock bound, so that a slow host can never cost the GPU line.
+    timeout_s=None: no bound, every one of `steps` is timed."""
+    budget = float('inf') if timeout_s is None else max(20.0, timeout_s - 40.0)
     cmd = [sys.executable, os.path.abspath(__file__), '--cpu-worker', '--steps', str(steps), '--warmup', str(warmup),
-           '--cpu-budget', str(max(20.0, timeout_s - 40.0))]
+           '--cpu-budget', str(budget)]
     try:
         out = subprocess.run(cmd, capture_output=True, text=True, timeout=timeout_s)
         for ln in reversed(out.stdout.strip().splitlines()):
@@ -204,6 +215,7 @@ def run_gpu(args):
     if world > 1:
         dist.init_process_group('nccl', device_id=dev)
     torch.manual_seed(0)
+    random.seed(0)      # the hyper-connections pick their initial stream with python's randrange (SURVEY A.5)
     tkw = dict(dim=cfg['dim'], depth=cfg['depth'], heads=cfg['heads'], dropout=args.dropout)
     B, N = cfg['batch'], cfg['seq']
     if kind == 'duration':
@@ -221,23 +233,39 @@ def run_gpu(args):
     text = [TEXT[i % 2] for i in range(B)]
     text_dev = pkg.list_str_to_tensor(text).to(dev)
     d2h_bytes = 4
+    last = {}     # --dump-outputs: what a recorded eager step returned (the loss detached: see GraphedTrainStep on eager outputs)
 
     if kind == 'sample':
         model.eval()
         d2h_bytes = B * N * 100 * 4
 
-        def step(mel, readback):
+        def step(mel, readback, record=False):
             out = model.sample(mel, text=text_dev, duration=N, steps=cfg['ode_steps'], cfg_strength=1.0, return_raw_output=True)
+            if record:
+                last['out'] = out
             return out.cpu() if readback else None
     else:
-        def step(mel, readback):
+        def step(mel, readback, record=False):
             loss = model(mel, text=text_dev) if kind == 'duration' else model(mel, text=text_dev).loss
             loss.backward()
             if sync is not None:
                 sync()
+            if record:
+                last['out'], last['grads'] = loss.detach(), [p.grad for p in model.parameters()]
             for p in model.parameters():
                 p.grad = None
             return loss.item() if readback else None
+
+    def outputs(out, grads=None):
+        """Host copies of one step's results for --dump-outputs (module docstring)."""
+        if grads is None:
+            return {'mel': out.float().cpu().numpy()}
+        params = list(model.parameters())
+        flat = torch.cat([(g if g is not None else torch.zeros_like(p)).detach().flatten().float() for p, g in zip(params, grads)])
+        idx = torch.randint(flat.numel(), (min(flat.numel(), 1 << 23),), generator=torch.Generator().manual_seed(0))
+        return {'loss': out.detach().float().reshape(1).cpu().numpy(),
+                'grad_norms': torch.stack([g.float().norm() if g is not None else torch.zeros((), device=dev) for g in grads]).cpu().numpy(),
+                'grads_sample': flat[idx.to(dev)].cpu().numpy()}
 
     def timed(fn, steps):
         if world > 1:
@@ -255,8 +283,8 @@ def run_gpu(args):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms) / steps
 
-    steps = args.steps if kind != 'sample' else max(1, min(args.steps, 3))   # one cfg5 step = 124 transformer forwards
-    warm = max(args.warmup, 3) if kind != 'sample' else 1
+    steps = args.steps
+    warm = max(args.warmup, 3) if kind != 'sample' else 1   # one cfg5 step = 124 transformer forwards
     for _ in range(warm):
         step(dev_mel, False)
     # -- time of the tcgen05 GEMM family inside one real step (roofline numerator / denominator): every ops.gemm call of ONE step is
@@ -303,8 +331,16 @@ def run_gpu(args):
     step_mode, graph_note, eager_ms = 'eager', None, None
     with ClockSampler(local) as clk:
         n0 = lib.launch_count()
-        ms_dev = timed(lambda: step(dev_mel, False), steps)
+        done = [0]
+
+        def dev_step():     # --dump-outputs: keep the results of the last timed step only, so that no earlier step's stay allocated
+            done[0] += 1
+            step(dev_mel, False, record=args.dump_outputs is not None and done[0] == steps)
+
+        ms_dev = timed(dev_step, steps)
         launches = (lib.launch_count() - n0) // steps
+        dumped = outputs(last['out'], last.get('grads')) if args.dump_outputs else None
+        last.clear()
         ms_e2e = timed(lambda: step(host_mel.to(dev, non_blocking=True), True), steps)
         ops.gemm = gemm_recorded
         nprof = 1
@@ -334,13 +370,14 @@ def run_gpu(args):
                 for _ in range(3):
                     graphed()
                 ms_g = timed(lambda: graphed(), steps)
+                dumped_g = outputs(graphed.out.loss, [p.grad for p in model.parameters()]) if args.dump_outputs else None
                 ms_g_e2e = timed(lambda: graphed(host_mel).item(), steps)
                 ok = torch.tensor([1.0 if ms_g < ms_dev else 0.0], device=dev)
                 if world > 1:
                     dist.all_reduce(ok, op=dist.ReduceOp.MIN)   # (both times are max-over-ranks already; keep the ranks in lockstep)
                 if float(ok) > 0:
                     eager_ms, step_mode = ms_dev, 'cuda_graph'
-                    ms_dev, ms_e2e, launches = ms_g, ms_g_e2e, graphed.launches_per_step
+                    ms_dev, ms_e2e, launches, dumped = ms_g, ms_g_e2e, graphed.launches_per_step, dumped_g
                 else:
                     graph_note = f'captured but not faster ({ms_g:.2f} ms)'
             except Exception as e:  # noqa: BLE001 - any capture problem: keep the eager measurement
@@ -387,6 +424,11 @@ def run_gpu(args):
     }
     if world == 1 and not args.no_cpu:
         line['cpu_baseline'] = run_cpu_bounded(steps=5, warmup=2, timeout_s=170.0)
+    if dumped is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), arr)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -404,7 +446,10 @@ def main():
     ap.add_argument('--no-graph', action='store_true', help='time the eager step only (skip the CUDA-graph replay of the same step)')
     ap.add_argument('--cpu-worker', action='store_true', help=argparse.SUPPRESS)
     ap.add_argument('--cpu-budget', type=float, default=150.0, help=argparse.SUPPRESS)
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step to DIR/<name>.npy (module docstring)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.cpu_worker:
         print(json.dumps(run_cpu(steps=args.steps, warmup=args.warmup, budget_s=args.cpu_budget)), flush=True)
         return
@@ -412,15 +457,14 @@ def main():
         if int(os.environ.get('RANK', '0')) != 0:
             return
         cfg = CONFIGS[args.config]
-        want = max(1, min(args.steps, 5))
-        r = run_cpu_bounded(steps=want, warmup=min(max(args.warmup, 1), 2), timeout_s=200.0)
+        r = run_cpu_bounded(steps=args.steps, warmup=min(max(args.warmup, 1), 2), timeout_s=None)
         print(json.dumps({
             'impl': 'reference', 'metric': METRIC, 'value': r['value'], 'unit': 'mel-frames/s', 'n_gpus': args.gpus, 'steps': r.get('timed_steps', 0),
             'warmup': min(max(args.warmup, 1), 2), 'ms_per_step': r.get('ms_per_step'), 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
             'dtype': 'f32', 'data': 'synthetic',
             'config': {'workload': cfg['name'], 'requested_steps': args.steps, 'requested_warmup': args.warmup,
                        'note': 'reference algorithm on the host CPU cores (oracle port), timed on BASELINE cfg1 = 2 of the 16 sequences of cfg2 per step '
-                               '(same model, same seq_len); each step is a bounded sample of the workload'},
+                               '(same model, same seq_len)'},
             'cpu_baseline': {k: r.get(k) for k in ('value', 'unit', 'cores', 'kind', 'sample')},
             'e2e': {'value': r['value'], 'unit': 'mel-frames/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}}))
         return

@@ -1,8 +1,8 @@
 """Load the reference's OWN e2_tts.py, unmodified, by file path (build container only).
 
-TEST INFRASTRUCTURE. `/root/reference` exists only in the build container, never on the GPU box, so
-this module is used exclusively by `oracle/make_golden.py` and by the CPU tests that pin
-`oracle/e2tts_oracle.py` against the reference (they skip when the reference tree is absent).
+TEST INFRASTRUCTURE. The reference tree is not part of this repository, so this module is used only
+by the scripts that mint the golden vectors under tests/golden/ (`oracle/make_golden.py`,
+`oracle/reference_cases.py`); the tests compare against those vectors.
 The reference's seven unvendored third-party imports resolve to `oracle/ref_leaves/` (restated
 semantics, SURVEY.md Appendix A) — `e2_tts_pytorch/__init__.py` is bypassed because it pulls in
 trainer.py -> matplotlib/accelerate which are not installed.
@@ -42,17 +42,23 @@ def load_reference():
 class TorchRecorder:
     """Proxy for the `torch` global inside the reference module: records the random draws of
     E2TTS.forward (e2_tts.py:1504 uniform_, :201 rand_like, :1519 randn_like, :1523 rand) so the
-    same (x0, times, span mask) can be injected into the oracle and the CUDA path."""
+    same (x0, times, span mask) can be injected into the oracle and the CUDA path. With `seed`, the randn_like
+    draws come from a torch.Generator seeded with it, so the first one can be redrawn without the reference."""
 
-    def __init__(self, torch_mod):
+    def __init__(self, torch_mod, seed=None):
         self._t = torch_mod
         self.log = {}
+        self._gen = None if seed is None else torch_mod.Generator().manual_seed(seed)
 
     def __getattr__(self, name):
         return getattr(self._t, name)
 
     def randn_like(self, *a, **k):
-        out = self._t.randn_like(*a, **k)
+        if self._gen is None:
+            out = self._t.randn_like(*a, **k)
+        else:
+            x = a[0]
+            out = self._t.randn(x.shape, generator=self._gen, dtype=x.dtype).to(x.device)
         self.log.setdefault('randn_like', []).append(out.clone())
         return out
 
@@ -62,10 +68,10 @@ class TorchRecorder:
         return out
 
 
-def run_reference_forward(ref, model, mel, text, lens=None, drop_text_cond=False):
+def run_reference_forward(ref, model, mel, text, lens=None, drop_text_cond=False, x0_seed=None):
     """Runs reference E2TTS.forward recording x0 / times / span mask. `drop_text_cond` is forced by
-    temporarily pinning cond_drop_prob (e2_tts.py:1261 uses python random())."""
-    rec = TorchRecorder(ref.torch)
+    temporarily pinning cond_drop_prob (e2_tts.py:1261 uses python random()). `x0_seed`: see TorchRecorder."""
+    rec = TorchRecorder(ref.torch, seed=x0_seed)
     span = {}
     orig_mffl = ref.mask_from_frac_lengths
 

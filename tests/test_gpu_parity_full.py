@@ -4,6 +4,7 @@ a d1024 / 16-head model — against the fp32 oracle (oracle/e2tts_oracle.py) com
 a sibling kernel. All calls go through the C ABI. Tolerances as in test_gpu_parity.py (bf16 tensor-core path vs fp32 oracle).
 """
 import math
+import random
 
 import pytest
 import torch
@@ -217,6 +218,7 @@ def test_attention_core_vs_fp32_softmax(pkg, Np, H, big_logits):
 # (a), (e) whole model at the BASELINE widths against the oracle run on the host CPU
 def _whole_model(pkg, tkw, B, N, lens, seed, tol_pred=3e-2, model_kw=None, e2tts_kw=None):
     torch.manual_seed(seed)
+    random.seed(seed)   # the hyper-connections pick their initial stream with python's randrange (SURVEY A.5): same model on every run
     model = pkg.E2TTS(transformer=dict(dropout=0., max_seq_len=N, **tkw, **(model_kw or {})), use_vocos=False, **(e2tts_kw or {}))
     # dyn_scale 0.05 (5x the reference's init of the hyper-connections' dynamic scales): with the 0.5 of the 2-layer fixtures a depth-8
     # stack amplifies bf16 rounding of the residual streams ~10x — the fp32 oracle with its OWN stage outputs rounded to bf16
@@ -305,6 +307,7 @@ def test_e2tts_interpolated_text_vs_oracle(pkg):
 # (f) sampling: euler, 32 steps, autoguidance null model — against the oracle's fixed-grid ODE on the host
 def _small_model(pkg, seed, depth=2):
     torch.manual_seed(seed)
+    random.seed(seed)   # the hyper-connections pick their initial stream with python's randrange (SURVEY A.5): same model on every run
     tkw = dict(dim=128, depth=depth, heads=2)
     model = pkg.E2TTS(transformer=dict(dropout=0., max_seq_len=256, **tkw), use_vocos=False)
     sd = O.randomize_zero_init({k: v.clone() for k, v in model.state_dict().items()}, seed=seed + 1)
